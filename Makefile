@@ -1,5 +1,7 @@
 # Builds libctr_b200.so (sm_100a only) in-tree; `python -c "import __graft_entry__ as g; g.build()"` calls this.
-NVCC      ?= nvcc
+CUDA_HOME ?= /usr/local/cuda
+# nvcc from PATH, else from the CUDA install (a plain user's PATH often lacks $(CUDA_HOME)/bin)
+NVCC      ?= $(if $(shell command -v nvcc),nvcc,$(CUDA_HOME)/bin/nvcc)
 ARCH      := -gencode arch=compute_100a,code=sm_100a
 NVCCFLAGS := -O3 -std=c++17 -lineinfo $(ARCH) -Xcompiler -fPIC,-Wall,-Wno-unused-function -Xptxas -v
 SRC_DIR   := tf_repos_b200/csrc

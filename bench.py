@@ -29,6 +29,8 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+# the tree this runs from may be read-only and stays as build() left it: no __pycache__ written from here
+sys.dont_write_bytecode = True
 
 CFG = dict(model="DeepFM", field_size=39, feature_size=200_000_000, embedding_size=16, batch_size=8192,
            deep_layers="256,128,64", dropout="0.5,0.5,0.5", l2_reg=1e-4, learning_rate=5e-4, optimizer="Adam")
@@ -52,7 +54,13 @@ def parse():
     ap.add_argument("--tables", default="auto", choices=["auto", "replicated", "sharded"],
                     help="N>1: 'sharded' = rows owned by id %% N, NCCL all-to-all exchange (default); "
                          "'replicated' = data parallel with all-gathered sparse gradients")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the headline timed steps, write what the last of them computed (loss terms, "
+                         "probabilities, dense variables, a seeded row sample of fm_v / fm_w) as DIR/<name>.npy")
+    a = ap.parse_args()
+    if a.dump_outputs and (a.impl != "b200" or int(os.environ.get("WORLD_SIZE", "1")) != 1):
+        ap.error("--dump-outputs needs the b200 arm on one GPU")
+    return a
 
 
 def peaks():
@@ -279,9 +287,11 @@ def main_b200(args):
             return model.train_step_graphed(ids, vals, labels)
         return model.train_step(ids, vals, labels)
 
+    last = {}
+
     def step_dev(i):
         ids, vals, labels = devb[i % N_BATCHES]
-        train(ids, vals, labels)
+        last["ids"], last["parts"] = ids, train(ids, vals, labels)
 
     counts = {}
     step_exact_marker = object()
@@ -331,6 +341,8 @@ def main_b200(args):
     sweep_steps = list(model.updater.sweep_steps)
     model.updater.sweep_events = None
     model.check_ids()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, model, last["parts"], last["ids"])
     ms_step = ms_total / args.steps
     value = world * B * args.steps / (ms_total * 1e-3)
 
@@ -577,6 +589,41 @@ def main_b200(args):
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
+
+
+DUMP_ROWS = 1 << 17  # table rows of each kind in --dump-outputs: rows the last step gathered, rows drawn at random
+
+
+def dump_outputs(out_dir, model, parts, ids):
+    """Writes what the last timed step computed as float32 / float64 DIR/<name>.npy (about 20 MB here; at most 64 MB).
+    Inputs, initial state and dropout masks follow from fixed seeds, so two builds run with the same arguments can be
+    compared file by file.  The 200M-row tables are sampled with a fixed seed: up to DUMP_ROWS rows the last step
+    gathered (their gradient moved them) plus DUMP_ROWS uniform rows (only the l2 term moved them)."""
+    import numpy as np
+    import torch
+
+    g = torch.Generator().manual_seed(0)
+
+    def sample(x, n):
+        return x if x.numel() <= n else x[torch.randperm(x.numel(), generator=g)[:n].sort().values]
+
+    variables = model.variables()
+    gathered = sample(torch.unique(ids.reshape(-1).long().cpu()), DUMP_ROWS)
+    rows = torch.unique(torch.cat([gathered, torch.randint(0, model.N, (DUMP_ROWS,), generator=g)]))
+    rows_dev = rows.to(model.device)
+    # the step's loss, left to right: mean CE, then the l2 terms of the tables, which the exact-deferred update
+    # computes in its sweep rather than in the step's returned tensor
+    pos = (model.epoch_pos - 1) % model.epoch_steps
+    n_tab = len(model.tables)
+    out = {"loss_terms": torch.cat([parts[:-n_tab], model.epoch_reg_terms()[:, pos]]),
+           "prob": sample(model.pred[: model.B].cpu(), 1 << 20),
+           "sample_rows": rows.double(),
+           "fm_v_sample_rows": variables["fm_v"][rows_dev],
+           "fm_w_sample_rows": variables["fm_w"][rows_dev]}
+    out.update({name.replace("/", "."): v for name, v in variables.items() if name not in ("fm_v", "fm_w")})
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), v.detach().cpu().numpy())
 
 
 def side_models(torch, dev, synth, vocab):
